@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- optimisation steps/sec of the Aphantasia hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): clip_fft.py --size 1280-720 --samples 200 ViT-B/32 FFT -> S = int(200*0.95) = 190
@@ -358,6 +358,8 @@ def run_ours(args):
     t_dev = timed(ds.step, K, Wm, barrier)
     launches = (_lib.lib().aph_launch_count() - l0) * K // (K + Wm)
     clk = clocks.stop() if clocks else None
+    if args.dump_outputs and rank == 0:       # before the stage timing below runs more steps on the same buffers
+        dump_outputs(ds, args.dump_outputs)
     # per-stage split + GEMM-kernel timing, measured live right after the timed region (same process, same buffers)
     ds.ev = []
     for i in range(3):
@@ -490,6 +492,16 @@ def run_ours(args):
     emit(out)
 
 
+def dump_outputs(ds, out_dir):
+    """Writes what the last timed step of the device leg handed back, one .npy per array (~34 MB at C2): the loss, the crop
+    embeddings (rank 0's shard when --gpus > 1), the RGB canvas, the spectrum gradient and the spectrum after that step's Adam
+    update. Inputs are seeded, so two builds run with the same arguments can be compared array for array."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {'loss': -ds.loss, 'embeddings': ds.emb, 'image': ds.rgb, 'spectrum_grad': ds.g_params, 'spectrum': ds.params}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().float().cpu().numpy())
+
+
 def time_gemms(ds, S):
     """Average duration of the step's tcgen05 GEMM launches: each shape of the step replayed on the handle's own
     operand-sized buffers with CUDA events on the launching stream (after warm-up)."""
@@ -584,7 +596,12 @@ def _main():
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--config', default='c2', choices=sorted(CONFIGS), help='c2 = the bench line (default); others: supplementary e2e runs')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write the outputs of the last one to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and (args.impl != 'ours' or args.config != 'c2'):
+        ap.error('--dump-outputs writes the outputs of the bench line: --impl ours --config c2')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
     if args.impl == 'ours' and args.config != 'c2':
         run_supplementary(args)

@@ -129,13 +129,13 @@ def main():
                                                        ('mid', (230, 260), 6, 224, 'uniform', 0.4, 9, 7),
                                                        ('over', (80, 120), 6, 32, 'overscan', 0.4, 13, 1)]:
         seed(100 + s)
-        canvas = torch.rand(1, 3, *hw).half().float().requires_grad_(True)   # fp16-exact values: stored compactly
+        canvas = torch.rand(1, 3, *hw).half().float().requires_grad_(True)   # stored as its seed: the tests redraw it
         seed(s)
         out = ref.utils.slice_imgs([canvas], cnt, size, fast, align, macro)[0]
         seed(200 + s)
         cot = torch.randn(out.shape)
         (out * cot).sum().backward()
-        g['smp_%s_canvas' % name] = canvas.detach().numpy().astype(np.float16)
+        g['smp_%s_canvas_seed' % name] = np.array(100 + s)
         g['smp_%s_cfg' % name] = np.array([hw[0], hw[1], cnt, size, macro, s, sub], np.float64)
         g['smp_%s_align' % name] = np.array(align)
         g['smp_%s_out' % name] = out.detach().numpy()[:, :, ::sub, ::sub]

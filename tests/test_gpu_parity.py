@@ -111,7 +111,8 @@ def test_sampler_vs_reference_golden(L, golden, name):
     H, W, cnt, size, macro, s, sub = (float(v) for v in golden['smp_%s_cfg' % name])
     H, W, cnt, size, s, sub = int(H), int(W), int(cnt), int(size), int(s), int(sub)
     align = str(golden['smp_%s_align' % name])
-    canvas = torch.tensor(golden['smp_%s_canvas' % name].astype(np.float32)).cuda().requires_grad_(True)
+    _seed(golden['smp_%s_canvas_seed' % name])
+    canvas = torch.rand(1, 3, H, W).half().float().cuda().requires_grad_(True)
     _seed(s)
     out = slice_imgs([canvas], cnt, size, transforms.transforms_fast, align, macro)[0]
     assert _rel(out[:, :, ::sub, ::sub], golden['smp_%s_out' % name]) < 1e-5
@@ -122,7 +123,7 @@ def test_sampler_vs_reference_golden(L, golden, name):
     assert _rel(canvas.grad[:, :, ::st, ::st], golden['smp_%s_gcanvas' % name]) < 1e-4
 
 
-def test_sampler_backward_variants_agree(L):
+def test_sampler_backward_variants_agree(L, tmp_path):
     """Backward variants (each in its own process): default = three-kernel form (rotation adjoint as a gather, 3 channels per thread);
     APH_SAMPLE_BWD_OLD=1 = one-kernel form, fp32 compare-and-swap shared accumulation; APH_SAMPLE_BWD_FIXED=1 = one-kernel form, integer
     fixed-point shared accumulation; APH_SAMPLE_BWD_GATHER=1 = atomic-free tile gather. All must agree to fp32 round-off, also
@@ -144,7 +145,7 @@ torch.save(c.grad.cpu(), sys.argv[1])
     for mag in ('1.0', '1e-6'):
         outs = []
         for k, env_add in enumerate((dict(APH_SAMPLE_BWD_FIXED='1'), dict(), dict(APH_SAMPLE_BWD_GATHER='1'), dict(APH_SAMPLE_BWD_OLD='1'))):
-            path = '/tmp/aph_bwd_variant_%d.pt' % k
+            path = str(tmp_path / ('variant_%d.pt' % k))
             subprocess.check_call([sys.executable, '-c', code, path, mag], env=dict(os.environ, **env_add))
             outs.append(torch.load(path))
         # the one-kernel variants share the forward's tap arithmetic; the default evaluates the rotation adjoint's weights from the

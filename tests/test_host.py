@@ -90,6 +90,7 @@ def _free_port():
 
 def _worker(rank, world, port, q):
     os.environ.update(RANK=str(rank), WORLD_SIZE=str(world), LOCAL_RANK=str(rank), MASTER_ADDR='127.0.0.1', MASTER_PORT=str(port))
+    torch.cuda.is_available = lambda: False      # the ranks act as GPU-less hosts (gloo), also where there are fewer GPUs than ranks
     sys.path.insert(0, ROOT)
     from aphantasia_b200 import _dist, _rng
     torch.manual_seed(100 + rank); np.random.seed(100 + rank)      # deliberately different before the seed sync
@@ -112,8 +113,13 @@ def test_two_rank_gloo_sharding_matches_single_process():
     q, port = ctx.Queue(), _free_port()
     procs = [ctx.Process(target=_worker, args=(r, 2, port, q)) for r in range(2)]
     for p in procs: p.start()
-    res = sorted(q.get(timeout=120) for _ in range(2))
-    for p in procs: p.join(30)
+    try:
+        res = sorted(q.get(timeout=120) for _ in range(2))
+    finally:
+        for p in procs:
+            p.join(30)
+            if p.is_alive():        # its peer died: it would wait in the rendezvous and keep pytest from exiting
+                p.terminate()
     (r0, t0, s0, g0, m0), (r1, t1, s1, g1, m1) = res
     assert t0 == t1, 'ranks replayed different random streams'
     assert s0 == (0, 6) and s1 == (6, 11)

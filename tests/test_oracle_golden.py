@@ -61,7 +61,8 @@ def test_sampler_oracle(golden, name):
     H, W, cnt, size, macro, s, sub = (float(v) for v in golden['smp_%s_cfg' % name])
     H, W, cnt, size, s, sub = int(H), int(W), int(cnt), int(size), int(s), int(sub)
     align = str(golden['smp_%s_align' % name])
-    canvas = torch.tensor(golden['smp_%s_canvas' % name].astype(np.float32)).requires_grad_(True)
+    _seed(golden['smp_%s_canvas_seed' % name])
+    canvas = torch.rand(1, 3, H, W).half().float().requires_grad_(True)
     _seed(s)
     tabs, frame = _rng.draw_crop_table(cnt, (H, W), size, _rng.TF_FAST, align, macro)
     out = R.sample_crops(canvas, tabs[0], size, 2, frame)
