@@ -46,6 +46,12 @@ _SIGS = {
     'aph_vit_fwd_prepatched': (C.c_int, [C.c_void_p, C.c_int, c_f32p, C.c_int, C.c_void_p]),
     'aph_vit_bwd': (C.c_int, [C.c_void_p, c_f32p, C.c_int, c_f32p, C.c_void_p]),
     'aph_vit_bytes': (C.c_int64, [C.c_void_p]),
+    'aph_text_create': (C.c_int, [C.POINTER(C.c_void_p), C.c_void_p]),
+    'aph_text_destroy': (C.c_int, [C.c_void_p]),
+    'aph_text_load_tensor': (C.c_int, [C.c_void_p, C.c_char_p, c_f32p, C.c_int64, C.c_void_p]),
+    'aph_text_finalize': (C.c_int, [C.c_void_p]),
+    'aph_text_fwd': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, c_f32p, C.c_void_p]),
+    'aph_text_bytes': (C.c_int64, [C.c_void_p]),
     'aph_gemm_bf16_tn': (C.c_int, [C.c_void_p, C.c_void_p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     'aph_gemm_epi_test': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, c_f32p, c_f32p, C.c_void_p, C.c_int, c_f32p, C.c_void_p, C.c_void_p,
                                     C.c_int, C.c_int, C.c_void_p]),
@@ -66,6 +72,10 @@ EXPORTS = tuple(_SIGS)
 
 class VitConfig(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ('patch', 'width', 'layers', 'heads', 'out_dim', 'res', 'max_batch', 'reserved')]
+
+
+class TextConfig(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ('width', 'layers', 'heads', 'ctx', 'vocab', 'out_dim', 'max_batch')]
 
 
 def lib():

@@ -152,7 +152,7 @@ __global__ void __launch_bounds__(256) k_pack_weight(const float* __restrict__ i
   }
 }
 
-static int pack(const float* src, bf16* dst, int rows, int cols, int transpose, cudaStream_t st) {
+int pack(const float* src, bf16* dst, int rows, int cols, int transpose, cudaStream_t st) {     // also text.cu
   const size_t n = (size_t)rows * cols;
   const int blocks = (int)std::min<size_t>((n + 255) / 256, (size_t)kNumSMs * 16);
   k_pack_weight<<<blocks, 256, 0, st>>>(src, dst, rows, cols, transpose);
@@ -164,17 +164,6 @@ static int copy_f32(const float* src, float* dst, size_t n, cudaStream_t st) {
   APH_CUDA_OK(cudaMemcpyAsync(dst, src, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return 0;
 }
-
-#define NCH_DISPATCH(D, ...)                                                           \
-  switch ((D) / 128) {                                                                 \
-    case 1: { constexpr int NCH = 1; __VA_ARGS__; } break;                             \
-    case 2: { constexpr int NCH = 2; __VA_ARGS__; } break;                             \
-    case 6: { constexpr int NCH = 6; __VA_ARGS__; } break;                             \
-    case 8: { constexpr int NCH = 8; __VA_ARGS__; } break;                             \
-    default: set_error("vit: unsupported width %d", (D)); return 2;                    \
-  }
-
-static inline int rows_grid(int rows) { return (rows * 32 + 255) / 256; }
 
 // APH_ATTN_SIMT=1 selects the fp32 SIMT attention kernels (debug / comparison); default = tensor-core kernels.
 static bool attn_simt() {
@@ -188,6 +177,21 @@ static bool attn_umma() {
   static int v = -1;
   if (v < 0) { const char* e = getenv("APH_ATTN_UMMA"); v = (e && e[0] == '0') ? 0 : 1; }
   return v == 1;
+}
+
+// Causal self-attention of the CLIP text tower (text.cu): the mma.sync forward with keys j > i masked, one CTA per
+// (sample, head), T = context length <= 112.
+int attn_fwd_causal(const bf16* qkv, bf16* out, int S, int T, int D, int heads, cudaStream_t st) {
+  APH_REQUIRE(T > 0 && T <= 112, "causal attention: T=%d outside (0, 112]", T);
+  constexpr size_t smem = attn_tc_fwd_smem<8, 7>();
+  static bool cfg = false;
+  if (!cfg) {
+    APH_CUDA_OK(cudaFuncSetAttribute(k_attn_fwd_tc<8, 7, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cfg = true;
+  }
+  APH_CUDA_OK(launch_k(k_attn_fwd_tc<8, 7, true>, dim3(S * heads), dim3(8 * 32), smem, st, 1, qkv, out, T, D, heads));
+  APH_LAUNCH_OK();
+  return 0;
 }
 
 }  // namespace aph

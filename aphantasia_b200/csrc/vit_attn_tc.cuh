@@ -80,7 +80,8 @@ __device__ __forceinline__ void av_step(float (&acc)[8][4], const uint32_t (&a)[
 }
 
 // ---------------------------------------------------------------------------------------------
-template <int NW, int NT2>
+// CAUSAL (the CLIP text tower): query row i sees keys j <= i only; key tiles wholly above the warp's rows are skipped.
+template <int NW, int NT2, bool CAUSAL = false>
 __global__ void __launch_bounds__(NW * 32) k_attn_fwd_tc(const bf16* __restrict__ qkv, bf16* __restrict__ out, int T, int D, int heads) {
   pdl_trigger(); pdl_wait();
   extern __shared__ __align__(128) uint8_t sm[];
@@ -108,11 +109,23 @@ __global__ void __launch_bounds__(NW * 32) k_attn_fwd_tc(const bf16* __restrict_
     float m0 = -INFINITY, m1 = -INFINITY;
 #pragma unroll
     for (int n2 = 0; n2 < NT2; ++n2) {
+      if (CAUSAL && n2 * 16 > q0 + r0 + 15) {          // every key of the tile lies above the diagonal of this warp's rows
+#pragma unroll
+        for (int u = 0; u < 2; ++u) c[2 * n2 + u][0] = c[2 * n2 + u][1] = c[2 * n2 + u][2] = c[2 * n2 + u][3] = -INFINITY;
+        continue;
+      }
       qk_tile(c[2 * n2], c[2 * n2 + 1], qa, ks_a, n2 * 16, lane);
 #pragma unroll
       for (int u = 0; u < 2; ++u) {
         const int col = n2 * 16 + u * 8 + 2 * t;
         float* cc = c[2 * n2 + u];
+        if (CAUSAL) {      // rows q0 + r0 + g and + 8 see keys j <= i; key 0 always, so m0, m1 stay finite
+          const int qi = q0 + r0 + g;
+          if (col > qi) cc[0] = -INFINITY;
+          if (col + 1 > qi) cc[1] = -INFINITY;
+          if (col > qi + 8) cc[2] = -INFINITY;
+          if (col + 1 > qi + 8) cc[3] = -INFINITY;
+        }
         cc[0] = (col < T) ? cc[0] * kAttnScaleLog2 : -INFINITY; cc[1] = (col + 1 < T) ? cc[1] * kAttnScaleLog2 : -INFINITY;
         cc[2] = (col < T) ? cc[2] * kAttnScaleLog2 : -INFINITY; cc[3] = (col + 1 < T) ? cc[3] * kAttnScaleLog2 : -INFINITY;
         m0 = fmaxf(m0, fmaxf(cc[0], cc[1])); m1 = fmaxf(m1, fmaxf(cc[2], cc[3]));
@@ -131,6 +144,7 @@ __global__ void __launch_bounds__(NW * 32) k_attn_fwd_tc(const bf16* __restrict_
     for (int i = 0; i < 8; ++i) { o[i][0] = o[i][1] = o[i][2] = o[i][3] = 0.f; }
 #pragma unroll
     for (int kk = 0; kk < NT2; ++kk) {
+      if (CAUSAL && kk * 16 > q0 + r0 + 15) continue;   // P is exactly zero there
       uint32_t pa[4] = {pack2(c[2 * kk][0], c[2 * kk][1]), pack2(c[2 * kk][2], c[2 * kk][3]),
                         pack2(c[2 * kk + 1][0], c[2 * kk + 1][1]), pack2(c[2 * kk + 1][2], c[2 * kk + 1][3])};
       av_step(o, pa, vs_a, kk * 16, lane);

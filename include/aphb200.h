@@ -176,6 +176,35 @@ int aph_vit_bwd(aph_vit* vit, const float* grad_emb, int S, float* grad_images, 
 /* bytes of device memory owned by the handle (weights + activation arena)                          */
 int64_t aph_vit_bytes(const aph_vit* vit);
 
+/* ================= CLIP text encoder (forward only) ===========================================
+ * Replaces clip.model.CLIP.encode_text (third-party OpenAI clip; call site clip_fft.py:150), run once per prompt
+ * before the optimisation loop:  x = token_embedding[ids] + positional_embedding;  `layers` residual attention
+ * blocks with a causal mask (query i sees keys j <= i);  emb = ln_final(x[s, argmax_t ids[s,t]]) @ text_projection.
+ * Same block as the image encoder (QuickGELU, LayerNorm eps 1e-5, head dim 64); the residual stream is fp32,
+ * GEMM operands bf16.                                                                                            */
+typedef struct aph_text aph_text;
+typedef struct {
+  int32_t width;      /* 256, 512 or 768 (ViT-B text towers: 512) */
+  int32_t layers;     /* 12                                        */
+  int32_t heads;      /* width / 64                                */
+  int32_t ctx;        /* context length, <= 112 (77)               */
+  int32_t vocab;      /* 49408                                     */
+  int32_t out_dim;    /* 512 (multiple of 128)                     */
+  int32_t max_batch;  /* largest n a call will pass                */
+} aph_text_config;
+int aph_text_create(aph_text** text, const aph_text_config* cfg);
+int aph_text_destroy(aph_text* text);
+/* One tensor of the OpenAI state dict by its key, without prefix ("token_embedding.weight", "positional_embedding",
+ * "ln_final.weight", "text_projection", "transformer.resblocks.3.attn.in_proj_weight", ...), fp32 DEVICE pointer.
+ * aph_text_finalize names the first tensor that never arrived.                                                    */
+int aph_text_load_tensor(aph_text* text, const char* key, const float* data, int64_t numel, void* stream);
+int aph_text_finalize(aph_text* text);
+/* tokens: int64 DEVICE [n, ctx] (clip.tokenize(...).cuda()) -> emb fp32 [n, out_dim]. An id outside [0, vocab)
+ * contributes a zero embedding row (the table is never read out of bounds).                                       */
+int aph_text_fwd(aph_text* text, const int64_t* tokens, int n, float* emb, void* stream);
+/* bytes of device memory owned by the handle (weights + activations)                                              */
+int64_t aph_text_bytes(const aph_text* text);
+
 /* Stand-alone tcgen05 GEMM used by the encoder (exported for tests / profiling):
  * C[M,N] (fp32) = A[M,K] (bf16, row-major) . B[N,K]^T (bf16, row-major). K % 64 == 0, N % 128 == 0. */
 int aph_gemm_bf16_tn(const void* A, const void* B, float* C, int M, int N, int K, void* stream);
